@@ -2,6 +2,7 @@
 """bench.py -- rays/sec of the SceneRF ray-render hot path on B200 (BASELINE.json metric), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload B|A|C] [--precision fp16|fp32]
+                    [--dump-outputs DIR]
 
 A "step" is one full render_rays_batch-equivalent pass (gaussian proposal MLP, sampling+sort, main MLP, compositing,
 RaySOM skipped as inference callers do, multi-GPU gather) over every ray of the workload:
@@ -10,6 +11,8 @@ Features and weights are packed and resident before the timed region (SURVEY.md 
 call; `e2e` times the reference-facing host-buffer call (pinned pixels H2D + depth/rgb D2H inside the timed region).
 N > 1 (torchrun): frame-per-GPU layout -- every rank renders its own full frame (own pose) and the packed depth+rgb
 of all frames are all-gathered over NCCL; per-GPU work is fixed => "scaling": "weak".
+--dump-outputs DIR writes what the last timed step returned.  Inputs, weights and noise seeds depend only on the
+arguments, so two builds run with the same arguments can be compared array by array.
 --impl reference times the CPU restatement of the reference (oracle/, pinned to the reference's own outputs) on the host
 cores with a process pool; the reference itself is PyTorch-on-Python and is not present on the GPU box.
 """
@@ -668,6 +671,28 @@ def time_loop(fn, steps, warmup, sync):
     return e0.elapsed_time(e1) / steps
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+NPY_HEADER_BYTES = 128
+
+
+def dump_outputs(path, arrays, ray_axis=0, limit_bytes=DUMP_LIMIT_BYTES, seed=0):
+    """--dump-outputs: every array of `arrays` (name -> tensor, rays along `ray_axis`) as path/<name>.npy in float32, so
+    that two builds can be compared output for output.  Above `limit_bytes` in all, every array keeps the same fixed,
+    seeded sample of rays (in ray order), whose indices are written as path/ray_index.npy (float64)."""
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[ray_axis]
+    per_ray = sum(a.nbytes for a in arrays.values()) // max(1, n)
+    budget = limit_bytes - NPY_HEADER_BYTES * (len(arrays) + 1)
+    if per_ray * n > budget:
+        keep = min(n, budget // (per_ray + 8))
+        idx = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        arrays = {k: np.take(a, idx, axis=ray_axis) for k, a in arrays.items()}
+        arrays["ray_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a))
+
+
 def max_over_ranks(ms, dev, world):
     import torch
     import torch.distributed as dist
@@ -813,8 +838,10 @@ def run_render(args, rank, world, local_rank):
             dist.barrier()
         torch.cuda.synchronize()
 
+    # `last` holds one step's outputs while the next step allocates its own, in the warm-up as in the timed loop, so that
+    # the timed steps reuse cached allocations
     for _ in range(args.warmup):
-        step_device()
+        last = step_device()
     sampler = ClockSampler(local_rank)
     barrier()
     sampler.start()
@@ -823,7 +850,7 @@ def run_render(args, rank, world, local_rank):
     launches = 0
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
         launches += r.last_launches
         mlp_ms.append(r.last_mlp_ms()[1])            # waits for this step's main-MLP end event only
     ev1.record()
@@ -831,6 +858,10 @@ def run_render(args, rank, world, local_rank):
     clocks = sampler.stop()
     ms_per_step = max_over_ranks(ev0.elapsed_time(ev1), dev, world) / args.steps
     value = world * R / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # one GPU: the dict render_rays_batch returns; N GPUs: the gathered (N, R, 4) [depth, r, g, b] frames
+        dump_outputs(args.dump_outputs, last if world == 1 else {"frames": last}, ray_axis=0 if world == 1 else 1)
+    del last
 
     # ---- e2e: host buffers in, host buffers out, through the reference-facing call ------------------------------
     out_host = {"depth": torch.empty((R,), dtype=torch.float32).pin_memory(),
@@ -1033,7 +1064,14 @@ def main():
     ap.add_argument("--latent-table", type=int, default=0, help="1: the timed renderer uses the pre-projected latent table (diagnostics / profiling)")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong-scaling / workload D / workload E measurements")
     ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer (e2e) loop; 0 = same as --steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (float32, at most "
+                         "64 MB in all: a fixed, seeded sample of rays beyond that); render workloads A, B, Bp and C")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("A", "B", "Bp", "C")):
+        ap.error("--dump-outputs applies to --impl ours with the render workloads A, B, Bp and C")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -603,6 +603,19 @@ def angles_kat():
     return out
 
 
+@case
+def reference_sources():
+    """sha256 of every reference file oracle/build_ref.py stages into oracle/_ref, so that a staged copy can be checked
+    on a machine without the reference tree."""
+    import hashlib
+    from oracle import build_ref
+    digests = []
+    for rel in build_ref.FILES:
+        with open(os.path.join(REF, rel), "rb") as f:
+            digests.append(hashlib.sha256(f.read()).hexdigest())
+    return {"files": np.array(build_ref.FILES), "sha256": np.array(digests)}
+
+
 def main():
     only = sys.argv[1:]
     for name, fn in CASES.items():
